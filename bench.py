@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — aligned query bp/s of the LexicMap query-side search path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4|c5] [--dump-outputs DIR]
 
 --config c2 (default; BASELINE.json configs[1], the driver's run): 10,000 synthetic 1-kb queries vs a 1,000-genome synthetic index
     (50 families x 20 members x 1 Mbp, SURVEY.md §8d generators, seeds 20260924/20260925), index written by lmi-tools with the reference's
@@ -12,9 +12,12 @@
     indexes and holds genomes [r*G/N, (r+1)*G/N), every rank searches the whole batch against its shard, per-query genome counts (`hits`)
     are summed with one NCCL all-reduce inside the timed region (what `lexicmap utils merge-search-results` does offline), e-values use the
     total bases of all shards. LMG_C3_GENOMES / LMG_C3_QUERIES scale it down for rehearsals (the JSON says so).
---config c4 (configs[3]): the reference's simulated ONT reads (tests/golden/demo_long_reads_sample.fasta.gz, 235 reads up to 90 kb; the full
-    demo/q.long-reads.fasta.gz when present) vs tests/data/demo.lmi with the reference's demo flags — the WFA-heavy path.
+--config c4 (configs[3]): the reference's simulated ONT reads (tests/golden/demo_long_reads_subset.fasta.gz, 31 reads up to 63 kb) vs
+    tests/data/demo.lmi (the demo genomes' windows of tests/golden/, seeded filler elsewhere) with the reference's demo flags — the WFA-heavy path.
 --config c5 (configs[4]): seed-lookup microbenchmark on a synthetic seeds-only image, range-partitioned by mask over the ranks.
+--dump-outputs DIR: after the timed steps, rank 0 writes what its last timed step returned as DIR/<name>.npy (float64): for c2-c4 every
+    numeric column of the HSP rows (hsp_<column>.npy; all rows up to 64 MB, else the rows of a seeded sample of whole queries) and the
+    rows per query; for c5 the lookup counters. The inputs are seeded, so two builds can be compared file by file.
 
 `value`   = sum of query bases / CUDA-event time of lmg_search_staged (queries already in HBM), max over ranks.
 `e2e`     = same metric through lmg_search_batch with HOST buffers (H2D of the queries and D2H of all rows inside the timed region).
@@ -229,6 +232,29 @@ def cpu_port_throughput(idx_dir, seqs, threads, target_s=12.0, params=None, whol
     return bp / dt, n, dt, len(rows)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_arrays(d, arrays):
+    os.makedirs(d, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), np.asarray(v, dtype=np.float64))
+
+
+def dump_rows(d, rows, nq):
+    """every numeric HSP column as float64 plus the rows per query; above DUMP_BYTES only the rows of whole queries, taken in a seeded order
+    while they fit, so that two builds with the same rows dump the same sample"""
+    names = [f for f in rows.dtype.names if f not in ("pad", "pad0", "cigar_off")]
+    per_q = np.bincount(rows["query"].astype(np.int64), minlength=nq)
+    budget = DUMP_BYTES - 8 * nq
+    if len(rows) * 8 * len(names) > budget:
+        order = np.random.default_rng(20260927).permutation(nq)
+        fits = order[np.cumsum(per_q[order]) * 8 * len(names) <= budget]
+        rows = rows[np.isin(rows["query"], fits)]
+    dump_arrays(d, dict({"rows_per_query": per_q}, **{"hsp_" + f: rows[f] for f in names}))
+    log("dumped %d rows (%d columns) to %s" % (len(rows), len(names), d))
+
+
 def cpu_desc(threads):
     n, total, quota = usable_cpus()
     return {"cores": threads, "cores_visible": total, "cores_usable": n, "cgroup_quota": quota}
@@ -308,13 +334,12 @@ def run_search(a, rank, world, local):
         idx_dir = DEMO_INDEX
         if not os.path.exists(os.path.join(idx_dir, "info.toml")):
             raise SystemExit("tests/data/demo.lmi is missing: run __graft_entry__.build() in the build container")
-        full = "/root/reference/demo/q.long-reads.fasta.gz"
-        qf = full if os.path.exists(full) else os.path.join(GOLD, "demo_long_reads_sample.fasta.gz")
+        qf = os.path.join(GOLD, "demo_long_reads_subset.fasta.gz")
         ids, seqs = read_fasta(qf)
-        rep = int(os.environ.get("LMG_C4_REPEAT", 8 if qf != full else 1))   # the 235-read sample is repeated so that a step is tens of Mbp
+        rep = int(os.environ.get("LMG_C4_REPEAT", 8))   # the sample is repeated so that a step holds enough work to time
         seqs = seqs * rep
         search_kw = dict(min_qcov_hsp=70.0, top_n_genomes=5, top_n_chains=1)
-        workload = "%d simulated ONT reads (%s x%d; 67-90,376 bp) vs the reference's 15 demo genomes, flags of demo/README.md:365-368; BASELINE.json configs[3] on the demo index" % (len(seqs), os.path.basename(qf), rep)
+        workload = "%d simulated ONT reads (%s x%d) vs the reference's 15 demo genomes (stored windows, seeded filler), flags of demo/README.md:365-368; BASELINE.json configs[3] on the demo index" % (len(seqs), os.path.basename(qf), rep)
         config = base_config(a, workload, {"queries_per_gpu": len(seqs), "genomes": 15, "masks": 20000, "sharding": "by query, index replicated" if a.gpus > 1 else "single GPU", "flags": search_kw})
         scaling = "weak"
     if cfgname != "c3":
@@ -355,20 +380,20 @@ def run_search(a, rank, world, local):
     launches0 = int(idx.timing()[1][15])
     ms_steps, stage_ms, probe_ms, nrows, wall_ms, e2e_lib_ms, e2e_stage, kern_ms, kcnt = [], np.zeros(8), [], 0, [], [], np.zeros(8), np.zeros(16), None
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    for _ in range(a.steps):
+    for i in range(a.steps):
         t = time.perf_counter()
-        r = idx.search_staged(staged, prm, collect="rows" if collect else False)
+        keep = collect or (a.dump_outputs and i == a.steps - 1)   # the rows are copied to the host after the library's timed region
+        r = idx.search_staged(staged, prm, collect="rows" if keep else False)
         ms, cnt = idx.timing()
         extra = 0.0
+        rows = r[0] if keep else None
+        nrows = len(rows) if keep else r
         if collect:
-            nrows = len(r[0])
             ev0.record()
-            hits_allreduce(r[0])
+            hits_allreduce(rows)
             ev1.record()
             torch.cuda.synchronize()
             extra = ev0.elapsed_time(ev1)
-        else:
-            nrows = r
         ms_steps.append(ms[7] + extra)
         stage_ms += ms[:8]
         probe_ms.append(ms[8])
@@ -376,6 +401,8 @@ def run_search(a, rank, world, local):
         kern_ms += ms
         kcnt = cnt
     sync_all()
+    if a.dump_outputs and rank == 0:
+        dump_rows(a.dump_outputs, rows, nq)
     launches = (int(idx.timing()[1][15]) - launches0) // max(a.steps, 1)
     # ---- e2e leg: host buffers in, rows out, every step
     e2e_ms = []
@@ -515,8 +542,12 @@ def run_c5(a, rank, world, local):
         dist.barrier()
     sampler = ClockSampler(local)
     sampler.start()
-    r = idx.probe_bench(nq, iters=max(a.steps, 1) + a.warmup)
+    if a.warmup:
+        idx.probe_bench(nq, iters=a.warmup)
+    r = idx.probe_bench(nq, iters=a.steps)   # after one untimed lookup pass of its own
     sampler.finish()
+    if a.dump_outputs and rank == 0:
+        dump_arrays(a.dump_outputs, {"probe_" + k: [r[k]] for k in ("issued", "survivors", "hits", "sum_log2", "sum_hit_sectors", "sum_values", "steps", "entries")})
 
     t = torch.tensor([r["survivors"], r["issued"], r["hits"], r["sum_log2"], r["sum_hit_sectors"], r["sum_values"], r["kernel_ms"], r["kernel_ms_best"], r["regroup_ms"]], device="cuda", dtype=torch.float64)
     if dist:
@@ -577,8 +608,7 @@ def run_reference(a):
     elif a.config == "c4":
         from conftest import DEMO_INDEX, GOLD
         idx_dir = DEMO_INDEX
-        full = "/root/reference/demo/q.long-reads.fasta.gz"
-        ids, seqs = read_fasta(full if os.path.exists(full) else os.path.join(GOLD, "demo_long_reads_sample.fasta.gz"))
+        ids, seqs = read_fasta(os.path.join(GOLD, "demo_long_reads_subset.fasta.gz"))
         search_kw = dict(min_qcov_hsp=70.0, top_n_genomes=5, top_n_chains=1)
         config = base_config(a, "simulated ONT reads vs the reference's 15 demo genomes (BASELINE.json configs[3] on the demo index)", {"genomes": 15, "flags": search_kw})
     else:
@@ -604,7 +634,10 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours")
     ap.add_argument("--config", default=os.environ.get("LMG_BENCH_CONFIG", "c2"), choices=["c2", "c3", "c4", "c5"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank, world, local = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     if a.impl == "reference":
         if rank == 0:

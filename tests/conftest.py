@@ -32,36 +32,73 @@ def make_queries(tmp, index, name, n, length, seed=20260925, max_sub=0.10, max_i
     return out
 
 
-DEMO_REFS = "/root/reference/demo/refs"          # only in the build container; the GPU box gets the prebuilt tests/data/demo.lmi
 DEMO_INDEX = os.path.join(ROOT, "tests", "data", "demo.lmi")
 GOLD = os.path.join(ROOT, "tests", "golden")
+DEMO_FILL_SEED = 20261017
+
+
+def write_demo_refs(out_dir):
+    """the reference's 15 demo genomes as the demo tests see them (tests/golden/demo_refs_windows.tsv.gz, made by
+    scripts/make_demo_fixture.py): every contig at its real length, the real bases in the stored windows around the HSPs the tests check,
+    seeded random bases everywhere else (one PCG64 stream over all contigs, so no two contigs share filler). Returns the FASTA paths."""
+    import gzip
+    import numpy as np
+    rng = np.random.PCG64(DEMO_FILL_SEED)   # the raw bit stream, which numpy keeps stable across versions
+    acgt = np.frombuffer(b"ACGT", np.uint8)
+
+    def filler(n):
+        b = rng.random_raw(n // 32 + 1).view(np.uint8)
+        return acgt[np.stack([b & 3, (b >> 2) & 3, (b >> 4) & 3, b >> 6], 1).reshape(-1)[:n]]
+    paths, f, seq = [], None, None
+
+    def flush():
+        if seq is not None:
+            f.write(b"%s\n" % seq.tobytes())
+    with gzip.open(os.path.join(GOLD, "demo_refs_windows.tsv.gz"), "rt") as src:
+        for line in src:
+            t = line.rstrip("\n").split("\t")
+            if t[0] == "G":
+                flush()
+                seq = None
+                if f:
+                    f.close()
+                paths.append(os.path.join(out_dir, t[1] + ".fa"))
+                f = open(paths[-1], "wb")
+            elif t[0] == "C":
+                flush()
+                f.write(b">%s\n" % t[1].encode())
+                seq = filler(int(t[2]))
+            else:
+                a = int(t[1])
+                seq[a:a + len(t[2])] = np.frombuffer(t[2].encode(), np.uint8)
+    flush()
+    f.close()
+    return paths
 
 
 def ensure_demo_index():
-    """index of the reference's 15 demo genomes (demo/refs) written by this repo's writer with the reference's default options
-    (20,000 masks, seed-desert filling). Built once in the build container (by __graft_entry__.build() or the first test that needs
-    it); `*.lmi/` is git-ignored but travels to the GPU box with the built .so files. Returns None when it cannot be provided."""
+    """index of the demo genomes (write_demo_refs) written by this repo's writer with the reference's default options (20,000 masks,
+    seed-desert filling). Built once, by __graft_entry__.build() or by the first test that needs it; tests/data/ is git-ignored."""
     if os.path.exists(os.path.join(DEMO_INDEX, "info.toml")):
         return DEMO_INDEX
-    if not os.path.isdir(DEMO_REFS):
-        return None
+    import shutil
+    import tempfile
     os.makedirs(os.path.dirname(DEMO_INDEX), exist_ok=True)
-    lst = DEMO_INDEX + ".list"
-    with open(lst, "w") as f:
-        f.write("\n".join(os.path.join(DEMO_REFS, x) for x in sorted(os.listdir(DEMO_REFS))) + "\n")
     tmp = DEMO_INDEX + ".tmp%d" % os.getpid()
-    subprocess.check_call([_tools(), "index", "--in-list", lst, "--out", tmp], stderr=subprocess.DEVNULL)
+    with tempfile.TemporaryDirectory() as d:
+        lst = os.path.join(d, "list")
+        with open(lst, "w") as f:
+            f.write("".join(p + "\n" for p in write_demo_refs(d)))
+        subprocess.check_call([_tools(), "index", "--in-list", lst, "--out", tmp], stderr=subprocess.DEVNULL)
+    if os.path.isdir(DEMO_INDEX):
+        shutil.rmtree(DEMO_INDEX)
     os.rename(tmp, DEMO_INDEX)
-    os.remove(lst)
     return DEMO_INDEX
 
 
 @pytest.fixture(scope="session")
 def demo_index():
-    d = ensure_demo_index()
-    if d is None:
-        pytest.skip("demo index not available (built in the build container from /root/reference/demo/refs)")
-    return d
+    return ensure_demo_index()
 
 
 def tsv_key(f):

@@ -71,13 +71,13 @@ def test_measurement_switches_do_not_change_a_byte(demo_index, tmp_path):
     """the environment switches that exist for A/B measurements (probe regrouping, L2 eviction hints, 16-bit anchor starts, lookup stream priority,
     the 128- and 256-diagonal register WFA kernels) select other kernels or layouts, never other results: the `-a` TSV of the simulated ONT reads
     (wide-band alignments included) is byte-identical under each of them"""
-    q = os.path.join(GOLD, "demo_long_reads_sample.fasta.gz")
+    q = os.path.join(GOLD, "demo_long_reads_subset.fasta.gz")
     def run(tag, extra):
         out = str(tmp_path / (tag + ".tsv"))
         subprocess.check_call([_cli(), "search", "-d", demo_index, q, "-o", out, "--quiet", "-a"], env=dict(os.environ, **extra))
         return open(out, "rb").read()
     base = run("default", {})
-    assert base.count(b"\n") > 200
+    assert base.count(b"\n") > 40
     for name in ("LMG_NO_REGROUP", "LMG_L2_HINTS", "LMG_CSTART32", "LMG_NO_PRIO_LOOKUP", "LMG_NO_WFA_REG8", "LMG_NO_WFA_REG"):
         assert run(name, {name: "1"}) == base, name
 

